@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- MD steps/s of the ViSNet energy/force hot path (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload chig]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload chig] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: neighbour build + ViSNet energy + analytic forces for
 every fragment of the protein + signed reduction to whole-protein energy/forces (what one MD step of the
@@ -49,7 +49,12 @@ def parse():
     ap.add_argument("--skip-cpu-baseline", action="store_true")
     ap.add_argument("--nccl", action="store_true", help="N > 1: torch.distributed all-reduce instead of the peer-memory one")
     ap.add_argument("--no-c4", action="store_true", help="N > 1: skip the 512-fragment strong-scaling leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the whole-protein forces and energy of the last timed step as DIR/forces.npy, DIR/energy.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed; it does not apply to --impl reference")
+    return args
 
 
 def load_workload(name, n_fragments=512):
@@ -305,6 +310,22 @@ def golden_reference(workload):
     return {"e": r[f"{workload}_ref_e"], "f": r[f"{workload}_ref_f"], "e64": r[f"{workload}_e64"], "f64": r[f"{workload}_f64"]}
 
 
+DUMP_FORCE_BYTES = 60 << 20          # keeps a dump under 64 MB
+
+
+def dump_outputs(out_dir, ef, n_protein):
+    """Write what a caller of the timed path (``vb_forward_protein``) receives, float32: ``forces.npy`` [n_protein, 3]
+    (eV/A) and ``energy.npy`` [1] (eV).  Forces above 60 MiB are a fixed sample of protein atoms, the rows
+    ``sort(default_rng(0).choice(n_protein, k, replace=False))``, so that two runs write the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    forces = ef[:-1].reshape(n_protein, 3)
+    if forces.nbytes > DUMP_FORCE_BYTES:
+        k = DUMP_FORCE_BYTES // forces[0].nbytes
+        forces = forces[np.sort(np.random.default_rng(0).choice(n_protein, k, replace=False))]
+    np.save(os.path.join(out_dir, "forces.npy"), forces)
+    np.save(os.path.join(out_dir, "energy.npy"), ef[-1:])
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -518,6 +539,8 @@ def run_ours(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ef.cpu().numpy(), pm.n_protein)
 
     # ---- per-kernel times + roofline (rank 0, its shard) ----
     n_edges = n_edges_local

@@ -277,6 +277,27 @@ def test_bench_roofline_arithmetic():
     assert b.tensor_roofline(["node_fwd0"], 1000, 1e-3, 3) is None
 
 
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: the whole-protein buffer [3*n + 1] as forces [n, 3] and energy [1], float32; forces over
+    the size limit as the same seeded sample of rows in every run."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    b = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(b)
+    ef = np.arange(3 * 50 + 1, dtype=np.float32)
+    b.dump_outputs(str(tmp_path / "full"), ef, 50)
+    f, e = np.load(tmp_path / "full" / "forces.npy"), np.load(tmp_path / "full" / "energy.npy")
+    assert f.dtype == np.float32 and np.array_equal(f, ef[:-1].reshape(50, 3))
+    assert e.dtype == np.float32 and e.tolist() == [150.0]
+    monkeypatch.setattr(b, "DUMP_FORCE_BYTES", 10 * 12)
+    b.dump_outputs(str(tmp_path / "s1"), ef, 50)
+    b.dump_outputs(str(tmp_path / "s2"), ef, 50)
+    s1, s2 = np.load(tmp_path / "s1" / "forces.npy"), np.load(tmp_path / "s2" / "forces.npy")
+    assert s1.shape == (10, 3) and np.array_equal(s1, s2)
+    rows = s1[:, 0].astype(np.int64) // 3
+    assert (np.diff(rows) > 0).all() and np.array_equal(s1, f[rows])
+
+
 @pytest.mark.parametrize("name", ["chig", "trpcage", "ww", "abd"])
 def test_fragment_membership_equals_the_reference_function(golden_dir, name):
     """Which protein atoms belong to every dipeptide / ACE-NME: the fixtures (ai2bmd_b200/pdbfrag.py) against the output
