@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -22,6 +23,7 @@
 #include "k_head.cuh"
 #include "k_md.cuh"
 #include "k_nonbonded.cuh"
+#include "k_restraint.cuh"
 #include "k_node.cuh"
 #include "k_node2.cuh"
 #include "k_node_tc.cuh"
@@ -191,6 +193,10 @@ struct vb_handle {
     float *d_nb_q = nullptr, *d_nb_sigma = nullptr, *d_nb_eps = nullptr;
     int *d_nb_rowptr = nullptr, *d_nb_col = nullptr;
     double* d_nb_eatom = nullptr;
+    // Hookean restraints (k_restraint.cuh)
+    bool rs_ready = false;
+    RsParams rs{};
+    void* rs_mem = nullptr;
 
     bool has_topology_sizes() const { return ws.N > 0; }
     void set_error(const char* fmt, ...) {
@@ -225,6 +231,10 @@ struct vb_handle {
         cudaFree(d_nb_q); cudaFree(d_nb_sigma); cudaFree(d_nb_eps); cudaFree(d_nb_rowptr); cudaFree(d_nb_col); cudaFree(d_nb_eatom);
         d_nb_q = d_nb_sigma = d_nb_eps = nullptr; d_nb_rowptr = d_nb_col = nullptr; d_nb_eatom = nullptr;
         nb_ready = false;
+    }
+    void free_rs() {
+        cudaFree(rs_mem);
+        rs_mem = nullptr; rs = RsParams{}; rs_ready = false;
     }
     void free_md() {
         cudaFree(d_mx); cudaFree(d_mv); cudaFree(d_mmass); cudaFree(d_ehist);
@@ -1034,6 +1044,7 @@ void vb_destroy(vb_handle* h) {
     cudaFree(h->d_tl);
     h->free_md();
     h->free_nb();
+    h->free_rs();
     h->free_comm();
     h->free_caph();
     cudaFree(h->arena);
@@ -1193,6 +1204,7 @@ int vb_set_protein_map(vb_handle* h, int64_t n_protein_atoms, int64_t n_map, con
     CUDA_TRY(h, cudaDeviceSynchronize());
     h->drop_graph();              // captured launches hold the old map pointers / n_protein
     h->free_md();                 // the MD state is sized by n_protein
+    h->free_rs();                 // ... and so are the restraints
     h->free_map();
     CUDA_TRY(h, cudaMalloc(&h->d_map_rowptr, sizeof(int) * (P + 1)));
     CUDA_TRY(h, cudaMalloc(&h->d_map_src, sizeof(int) * src.size()));
@@ -1228,7 +1240,7 @@ StepIO md_io(vb_handle* h) {
     io.ef = h->md_ef;
     return io;
 }
-// fragment placement -> evaluation + signed whole-protein reduction [-> non-bonded term], all on st
+// fragment placement -> evaluation + signed whole-protein reduction [-> non-bonded term] [-> restraints], all on st
 int md_eval_enqueue(vb_handle* h, cudaStream_t st) {
     const int N = h->ws.N;
     md_place_kernel<<<(N + 255) / 256, 256, 0, st>>>(N, h->d_real, h->d_acc, h->d_rem, h->d_blen, h->d_mx, h->d_pos);
@@ -1238,6 +1250,8 @@ int md_eval_enqueue(vb_handle* h, cudaStream_t st) {
         nonbonded_kernel<double><<<(h->nb.hi - h->nb.lo + 7) / 8, 256, 0, st>>>(h->nb, h->d_mx, h->md_ef, h->d_nb_eatom);
         nonbonded_energy_kernel<<<1, 256, 0, st>>>(h->nb, h->d_nb_eatom, h->md_ef);
     }
+    if (h->rs_ready && h->rs.hi > h->rs.lo)         // Hookean restraints on the same protein coordinates
+        restraint_kernel<<<1, RS_THREADS, 0, st>>>(h->rs, h->d_mx, h->md_ef);
     CUDA_TRY(h, cudaGetLastError());
     if (h->comm_ready && h->comm_auto) return enqueue_allreduce(h, st, h->md_ef, 3LL * h->n_protein + 1);
     return VB_OK;
@@ -1466,6 +1480,90 @@ int vb_nonbonded(vb_handle* h, const float* prot_pos_dev, float* ef_prot_dev, vo
         nonbonded_kernel<float><<<(h->nb.hi - h->nb.lo + 7) / 8, 256, 0, st>>>(h->nb, prot_pos_dev, ef_prot_dev, h->d_nb_eatom);
         nonbonded_energy_kernel<<<1, 256, 0, st>>>(h->nb, h->d_nb_eatom, ef_prot_dev);
     }
+    CUDA_TRY(h, cudaGetLastError());
+    return VB_OK;
+}
+
+
+// ---- Hookean restraints (k_restraint.cuh) ------------------------------------------------------------------------
+int vb_set_restraints(vb_handle* h, const vb_restraint_set* rs) {
+    if (!h) return VB_ERR_ARG;
+    std::lock_guard<std::mutex> lk(h->mu);
+    if (h->n_protein <= 0) { h->set_error("vb_set_restraints: call vb_set_protein_map first"); return VB_ERR_STATE; }
+    if (!rs) { h->set_error("vb_set_restraints: null restraint set"); return VB_ERR_ARG; }
+    const int P = h->n_protein;
+    const int64_t np_ = rs->n_point, nq = rs->n_pair;
+    auto bad = [&](const char* fmt, long long i) { h->set_error(fmt, i); return VB_ERR_ARG; };
+    if (np_ < 0 || nq < 0 || np_ + nq > (1 << 29)) return bad("vb_set_restraints: bad restraint count (%lld)", (long long)(np_ + nq));
+    if (rs->atom_lo < 0 || rs->atom_hi < rs->atom_lo || rs->atom_hi > P)
+        return bad("vb_set_restraints: bad slice: [atom_lo, atom_hi) must lie in [0, %lld)", (long long)P);
+    if ((np_ > 0 && (!rs->point_atom || !rs->point_anchor || !rs->point_k || !rs->point_rt)) ||
+        (nq > 0 && (!rs->pair_ij || !rs->pair_k || !rs->pair_rt)))
+        return bad("vb_set_restraints: null array for %lld restraints", (long long)(np_ + nq));
+    auto finite_nonneg = [](double v) { return std::isfinite(v) && v >= 0.0; };
+    for (int64_t i = 0; i < np_; i++) {
+        if (rs->point_atom[i] < 0 || rs->point_atom[i] >= P) return bad("vb_set_restraints: point restraint %lld: atom index out of range", (long long)i);
+        if (!finite_nonneg(rs->point_k[i]) || !finite_nonneg(rs->point_rt[i]))
+            return bad("vb_set_restraints: point restraint %lld: k and rt must be finite and non-negative", (long long)i);
+        for (int c = 0; c < 3; c++)
+            if (!std::isfinite(rs->point_anchor[3 * i + c])) return bad("vb_set_restraints: point restraint %lld: non-finite anchor", (long long)i);
+    }
+    for (int64_t q = 0; q < nq; q++) {
+        const int i = rs->pair_ij[2 * q], j = rs->pair_ij[2 * q + 1];
+        if (i < 0 || i >= P || j < 0 || j >= P) return bad("vb_set_restraints: pair restraint %lld: atom index out of range", (long long)q);
+        if (i == j) return bad("vb_set_restraints: pair restraint %lld: i == j", (long long)q);
+        if (!finite_nonneg(rs->pair_k[q]) || !finite_nonneg(rs->pair_rt[q]))
+            return bad("vb_set_restraints: pair restraint %lld: k and rt must be finite and non-negative", (long long)q);
+    }
+    // CSR over destination atoms, entries in restraint-id order within a row
+    std::vector<int> row(P + 1, 0);
+    for (int64_t i = 0; i < np_; i++) row[rs->point_atom[i] + 1]++;
+    for (int64_t q = 0; q < 2 * nq; q++) row[rs->pair_ij[q] + 1]++;
+    for (int a = 0; a < P; a++) row[a + 1] += row[a];
+    std::vector<int> ent(std::max<int64_t>(row[P], 1)), fill(row.begin(), row.end() - 1);
+    for (int64_t i = 0; i < np_; i++) ent[fill[rs->point_atom[i]]++] = (int)(2 * i);
+    for (int64_t q = 0; q < nq; q++) {
+        const int id = (int)(np_ + q);
+        ent[fill[rs->pair_ij[2 * q]]++] = 2 * id;
+        ent[fill[rs->pair_ij[2 * q + 1]]++] = 2 * id + 1;
+    }
+    // MD graph replays enqueued before this call may still read the old arrays
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    CUDA_TRY(h, cudaDeviceSynchronize());
+    h->drop_graph();
+    h->free_rs();
+    if (np_ == 0 && nq == 0) return VB_OK;            // empty set: the term is removed
+    struct Piece { const void* src; size_t bytes; size_t off; };
+    std::vector<Piece> pieces;
+    size_t total = 0;
+    auto add = [&](const void* src, size_t bytes) {
+        pieces.push_back({src, bytes, total});
+        total += (std::max<size_t>(bytes, 8) + 255) & ~(size_t)255;
+        return pieces.size() - 1;
+    };
+    const size_t i_row = add(row.data(), sizeof(int) * row.size()), i_ent = add(ent.data(), sizeof(int) * ent.size());
+    const size_t i_pa = add(rs->point_anchor, 24 * (size_t)np_), i_pk = add(rs->point_k, 8 * (size_t)np_), i_pr = add(rs->point_rt, 8 * (size_t)np_);
+    const size_t i_qij = add(rs->pair_ij, 8 * (size_t)nq), i_qk = add(rs->pair_k, 8 * (size_t)nq), i_qr = add(rs->pair_rt, 8 * (size_t)nq);
+    CUDA_TRY(h, cudaMalloc(&h->rs_mem, total));
+    char* base = static_cast<char*>(h->rs_mem);
+    for (const Piece& pc : pieces)
+        if (pc.bytes) CUDA_TRY(h, cudaMemcpy(base + pc.off, pc.src, pc.bytes, cudaMemcpyHostToDevice));
+    auto ip = [&](size_t i) { return reinterpret_cast<const int*>(base + pieces[i].off); };
+    auto dp = [&](size_t i) { return reinterpret_cast<const double*>(base + pieces[i].off); };
+    h->rs = RsParams{P, (int)rs->atom_lo, (int)rs->atom_hi, (int)np_, ip(i_row), ip(i_ent), dp(i_pa), dp(i_pk), dp(i_pr),
+                     ip(i_qij), dp(i_qk), dp(i_qr)};
+    h->rs_ready = true;
+    return VB_OK;
+}
+
+int vb_restraints(vb_handle* h, const double* prot_pos_dev, float* ef_prot_dev, void* stream) {
+    if (!h) return VB_ERR_ARG;
+    std::lock_guard<std::mutex> lk(h->mu);
+    if (h->n_protein <= 0) { h->set_error("vb_restraints: call vb_set_protein_map first"); return VB_ERR_STATE; }
+    if (!prot_pos_dev || !ef_prot_dev) { h->set_error("vb_restraints: null buffer"); return VB_ERR_ARG; }
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    if (h->rs_ready && h->rs.hi > h->rs.lo)
+        restraint_kernel<<<1, RS_THREADS, 0, (cudaStream_t)stream>>>(h->rs, prot_pos_dev, ef_prot_dev);
     CUDA_TRY(h, cudaGetLastError());
     return VB_OK;
 }
@@ -1727,6 +1825,7 @@ int64_t vb_get_option(const vb_handle* h, const char* key) {
         return v;
     }
     if (k == "comm_ready") return h->comm_ready ? 1 : 0;
+    if (k == "restraints_ready") return h->rs_ready ? 1 : 0;
     if (k == "edge_overflow") {
         int flag = 0;
         if (h->d_flags && cudaMemcpy(&flag, h->d_flags, sizeof(int), cudaMemcpyDeviceToHost) != cudaSuccess) return VB_ERR_CUDA;

@@ -34,13 +34,19 @@ class _CaphProblem(C.Structure):
                 ("lr", C.c_float), ("tol_grad", C.c_float), ("tol_change", C.c_float)]
 
 
+class _RestraintSet(C.Structure):
+    _fields_ = [("n_point", C.c_int64), ("point_atom", C.c_void_p), ("point_anchor", C.c_void_p), ("point_k", C.c_void_p),
+                ("point_rt", C.c_void_p), ("n_pair", C.c_int64), ("pair_ij", C.c_void_p), ("pair_k", C.c_void_p),
+                ("pair_rt", C.c_void_p), ("atom_lo", C.c_int64), ("atom_hi", C.c_int64)]
+
+
 # every symbol include/visnet_b200.h declares (tests check that the library exports each of them)
 EXPORTED_SYMBOLS = [
     "vb_weight_manifest", "vb_create", "vb_destroy", "vb_last_error", "vb_set_topology", "vb_forward",
     "vb_forward_host", "vb_set_protein_map", "vb_forward_protein", "vb_get_edges", "vb_launches_per_forward",
     "vb_set_option", "vb_get_option", "vb_num_stages", "vb_stage_name", "vb_debug_run", "vb_debug_read", "vb_profile_stages", "vb_tc_selftest",
     "vb_md_setup", "vb_md_set_normals", "vb_md_set_state", "vb_md_kick1", "vb_md_eval", "vb_md_kick2", "vb_md_run", "vb_md_get_state",
-    "vb_set_nonbonded", "vb_nonbonded",
+    "vb_set_nonbonded", "vb_nonbonded", "vb_set_restraints", "vb_restraints",
     "vb_comm_init", "vb_comm_connect", "vb_comm_allreduce",
     "vb_set_caph", "vb_caph_relax",
 ]
@@ -110,6 +116,10 @@ def load_library(path: Optional[str] = None):
     lib.vb_set_nonbonded.argtypes = [vp, i64, vp, vp, vp, vp, vp, i64, i64]
     lib.vb_nonbonded.restype = C.c_int
     lib.vb_nonbonded.argtypes = [vp, vp, vp, vp]
+    lib.vb_set_restraints.restype = C.c_int
+    lib.vb_set_restraints.argtypes = [vp, C.POINTER(_RestraintSet)]
+    lib.vb_restraints.restype = C.c_int
+    lib.vb_restraints.argtypes = [vp, vp, vp, vp]
     lib.vb_comm_init.restype = C.c_int
     lib.vb_comm_init.argtypes = [vp, C.c_int, C.c_int, i64, vp]
     lib.vb_comm_connect.restype = C.c_int
@@ -273,6 +283,32 @@ class Engine:
 
     def nonbonded_device(self, prot_pos_ptr: int, ef_ptr: int, stream_ptr: int = 0):
         self._check(self.lib.vb_nonbonded(self.h, prot_pos_ptr, ef_ptr, stream_ptr), "vb_nonbonded")
+
+    # ---- Hookean restraints (include/visnet_b200.h: vb_set_restraints / vb_restraints) ----
+    def set_restraints(self, point_atom=(), point_anchor=(), point_k=(), point_rt=(), pair_ij=(), pair_k=(), pair_rt=(),
+                       atom_lo: int = 0, atom_hi: int = -1):
+        """Install a restraint set (eV/A^2, A); replaces the previous one.  ``atom_hi < 0`` means every protein atom.
+        :class:`ai2bmd_b200.restraints.RestraintSet` holds these arrays (``RestraintSet.install(engine)``)."""
+        pa = np.ascontiguousarray(point_atom, dtype=np.int32).reshape(-1)
+        px = np.ascontiguousarray(point_anchor, dtype=np.float64).reshape(-1, 3)
+        pk = np.ascontiguousarray(point_k, dtype=np.float64).reshape(-1)
+        pr = np.ascontiguousarray(point_rt, dtype=np.float64).reshape(-1)
+        qij = np.ascontiguousarray(pair_ij, dtype=np.int32).reshape(-1, 2)
+        qk = np.ascontiguousarray(pair_k, dtype=np.float64).reshape(-1)
+        qr = np.ascontiguousarray(pair_rt, dtype=np.float64).reshape(-1)
+        if not (len(pa) == len(px) == len(pk) == len(pr) and len(qij) == len(qk) == len(qr)):
+            raise ValueError("restraint arrays have inconsistent lengths")
+        ptr = lambda a: a.ctypes.data if a.size else None
+        rs = _RestraintSet(len(pa), ptr(pa), ptr(px), ptr(pk), ptr(pr), len(qij), ptr(qij), ptr(qk), ptr(qr),
+                           int(atom_lo), int(self.n_protein if atom_hi < 0 else atom_hi))
+        self._check(self.lib.vb_set_restraints(self.h, C.byref(rs)), "vb_set_restraints")
+
+    def clear_restraints(self):
+        self.set_restraints()
+
+    def restraints_device(self, prot_pos_ptr: int, ef_ptr: int, stream_ptr: int = 0):
+        """ef[3n+1] += restraint forces / energy at the fp64 protein positions (device pointers); asynchronous."""
+        self._check(self.lib.vb_restraints(self.h, prot_pos_ptr, ef_ptr, stream_ptr), "vb_restraints")
 
     # ---- device-resident MD (include/visnet_b200.h: vb_md_*) ----
     def md_setup(self, masses, real, acc, rem, blen, dt, kT, friction, seed, ef_ptr: int):

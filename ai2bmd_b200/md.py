@@ -10,7 +10,8 @@ App. C) in numpy around :class:`BondedForceField`, which performs per step exact
   -> engine (energies/forces of every fragment) -> signed reduction to whole-protein energy / forces.
 
 friction = 0 gives velocity Verlet; its energy conservation is a physics check of the analytic forces
-(``tests/test_md_gpu.py``).  Units follow ASE: eV, Angstrom, amu, time in Angstrom*sqrt(amu/eV).
+(``tests/test_md_gpu.py``).  The reference's pre-equilibration and ``--constraints`` springs (ASE ``Hookean``) are
+:mod:`ai2bmd_b200.restraints`: ``DeviceLangevin.set_restraints`` on the device, a wrapped ``force_fn`` on the host.  Units follow ASE: eV, Angstrom, amu, time in Angstrom*sqrt(amu/eV).
 """
 from __future__ import annotations
 
@@ -192,6 +193,10 @@ class DeviceLangevin:
             if zero_com_momentum:
                 velocities -= (velocities * m).sum(0) / m.sum()
         engine.md_set_state(x, velocities, 0)
+        from .restraints import RestraintSet
+        self.restraints = RestraintSet()
+        if engine.get_option("restraints_ready"):          # a caller-supplied engine may carry a set: start without one
+            engine.clear_restraints()
         self._eval()
 
     @property
@@ -204,6 +209,20 @@ class DeviceLangevin:
         self.engine.md_eval(sp)
         if self.group is not None and not self._native_comm:
             self.torch.distributed.all_reduce(self.ef, group=self.group)
+
+    def set_restraints(self, rs):
+        """Make ``rs`` (an :class:`ai2bmd_b200.restraints.RestraintSet`, or None for none) the restraint term of every
+        following evaluation and recompute the forces at the current positions, so the next half-kick already uses it.
+        With ``group`` every rank computes the forces of an even slice of the protein atoms; the all-reduce sums them."""
+        from .restraints import RestraintSet
+        rs = RestraintSet() if rs is None else rs
+        dev = rs
+        if self.group is not None:
+            rank, world = self.torch.distributed.get_rank(self.group), self.torch.distributed.get_world_size(self.group)
+            dev = rs.sliced(rank * self.n // world, (rank + 1) * self.n // world)
+        dev.install(self.engine)
+        self.restraints = rs
+        self._eval()
 
     def set_normals(self, pool):
         """Externally supplied normals ``[steps, 2, n, 3]`` (float64) instead of the Philox stream (tests)."""

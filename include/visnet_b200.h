@@ -84,7 +84,8 @@ int vb_forward_protein(vb_handle* h, const float* pos_dev, float* ef_prot_dev, v
 
 /* ---- Device-resident MD step (SURVEY section 8f, rank 3 and the first half of rank 1) ------------------------
  * State (protein positions / velocities, fp64) stays on the GPU; one step is
- *   kick1 (half-kick + drift) -> eval (place fragment atoms, ViSNet, signed reduction into ef) -> kick2.
+ *   kick1 (half-kick + drift) -> eval (place fragment atoms, ViSNet, signed reduction into ef [+ non-bonded term]
+ *   [+ restraints]) -> kick2.
  * Replaces: the ASE Langevin loop the reference runs (src/AIMD/simulator.py:96-137: Langevin(dt = 1 fs, 300 K,
  *           friction 0.001/fs), MaxwellBoltzmannDistribution start; ASE 3.22 ase/md/langevin.py step()) and the
  *           per-step fragment coordinate rebuild with cap hydrogens on the acceptor->removed ray
@@ -132,6 +133,30 @@ int vb_set_nonbonded(vb_handle* h, int64_t n_protein_atoms, const float* charges
  * bonded + non-bonded (FragmentCalculator.calculate, src/Calculators/fragment.py:50-68).  Once set, vb_md_eval
  * adds the term too. */
 int vb_nonbonded(vb_handle* h, const float* prot_pos_dev, float* ef_prot_dev, void* stream);
+
+/* ---- Hookean restraints (pre-equilibration and hydrogen-bond constraints) ------------------------------------------
+ * point (a, p0, k, rt): d = p0 - x_a, r = |d|; if r > rt: F_a += k (r - rt) d/r, E += k (r - rt)^2 / 2.
+ * pair (i, j, k, rt):   d = x_j - x_i, r = |d|; if r > rt: F_i += k (r - rt) d/r, F_j -= k (r - rt) d/r, E += same.
+ * k in eV/Angstrom^2, rt and anchors in Angstrom; no periodic images.  Anchors are fixed copies, they do not follow the
+ * atom.  [atom_lo, atom_hi) are the destination atoms this handle computes (a sharded run gives every rank a slice and
+ * all-reduces the buffer); a restraint's energy is counted where its first atom is computed.
+ * Replaces: ASE 3.22 ase/constraints.py Hookean (adjust_forces / adjust_potential_energy) as the reference uses it:
+ *           position restraints of the pre-equilibration (src/AIMD/simulator.py:139-166) and the hydrogen-bond springs
+ *           of --constraints (simulator.py:168-180, pairs from PDBAnalyzer.find_bonded_atoms, src/utils/utils.py:169-221).
+ *           Host helpers that build the sets: ai2bmd_b200/restraints.py. */
+typedef struct {
+    int64_t n_point; const int32_t* point_atom; const double* point_anchor /*[n][3]*/; const double* point_k; const double* point_rt;
+    int64_t n_pair;  const int32_t* pair_ij /*[n][2]*/; const double* pair_k; const double* pair_rt;
+    int64_t atom_lo, atom_hi;
+} vb_restraint_set;
+/* Host pointers, copied.  Requires vb_set_protein_map (which drops the set again).  Both counts 0 removes the term.
+ * VB_ERR_ARG for an atom index outside [0, n_protein), i == j in a pair, a negative or non-finite k or rt, a non-finite
+ * anchor or a bad slice.  Synchronises the device before it replaces the arrays; captured graphs are dropped.  Once set,
+ * vb_md_eval / vb_md_run add the term after the bonded and non-bonded terms (before the automatic all-reduce). */
+int vb_set_restraints(vb_handle* h, const vb_restraint_set* rs);
+/* ef_prot_dev[3*n + 1] += restraint forces / energy at prot_pos_dev[n*3] (fp64 positions); adds nothing while no
+ * restraints are set.  Two calls on the same input give bit-identical results (no atomics). */
+int vb_restraints(vb_handle* h, const double* prot_pos_dev, float* ef_prot_dev, void* stream);
 
 /* ---- Per-step refinement of the added (cap) hydrogens (SURVEY section 8f, rank 1) -----------------------------------
  * One LBFGS call (lr, max_iter, tolerance_grad, tolerance_change; no line search, fresh state) on the Amber energy of all
@@ -189,7 +214,8 @@ int vb_launches_per_forward(const vb_handle* h);
  * fewest that fit one wave), "krot" 0/1 every CTA of the SIMT node kernels walks the K dimension of its weight chunks from a
  * different row (default 1: the CTAs of a wave otherwise ask the same L2 slices for the same rows at the same time),
  * "embed_batch" -1/0..3 batch variants of the embedding kernels, "comm_auto" 0/1.  vb_get_option also answers "edge_overflow" (1 after a step exceeded a trimmed max_edges),
- * "tile_rows" (planned edges per tile), "comm_ready", "caph_ready" and "caph_evals" (energy evaluations of the last hydrogen refinement). */
+ * "tile_rows" (planned edges per tile), "comm_ready", "caph_ready", "caph_evals" (energy evaluations of the last hydrogen refinement)
+ * and "restraints_ready" (1 while a non-empty restraint set is installed). */
 int vb_set_option(vb_handle* h, const char* key, int64_t value);
 int64_t vb_get_option(const vb_handle* h, const char* key);   /* resolved value (after vb_set_topology) */
 
