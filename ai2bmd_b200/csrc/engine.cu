@@ -23,6 +23,7 @@
 #include "k_head.cuh"
 #include "k_md.cuh"
 #include "k_nonbonded.cuh"
+#include "k_pme.cuh"
 #include "k_restraint.cuh"
 #include "k_node.cuh"
 #include "k_node2.cuh"
@@ -193,6 +194,10 @@ struct vb_handle {
     float *d_nb_q = nullptr, *d_nb_sigma = nullptr, *d_nb_eps = nullptr;
     int *d_nb_rowptr = nullptr, *d_nb_col = nullptr;
     double* d_nb_eatom = nullptr;
+    // PME non-bonded term (k_pme.cuh); at most one of nb_ready / pme_ready is set
+    bool pme_ready = false;
+    PmeParams pme{};
+    void* pme_mem = nullptr;
     // Hookean restraints (k_restraint.cuh)
     bool rs_ready = false;
     RsParams rs{};
@@ -231,6 +236,10 @@ struct vb_handle {
         cudaFree(d_nb_q); cudaFree(d_nb_sigma); cudaFree(d_nb_eps); cudaFree(d_nb_rowptr); cudaFree(d_nb_col); cudaFree(d_nb_eatom);
         d_nb_q = d_nb_sigma = d_nb_eps = nullptr; d_nb_rowptr = d_nb_col = nullptr; d_nb_eatom = nullptr;
         nb_ready = false;
+    }
+    void free_pme() {
+        cudaFree(pme_mem);
+        pme_mem = nullptr; pme = PmeParams{}; pme_ready = false;
     }
     void free_rs() {
         cudaFree(rs_mem);
@@ -1044,6 +1053,7 @@ void vb_destroy(vb_handle* h) {
     cudaFree(h->d_tl);
     h->free_md();
     h->free_nb();
+    h->free_pme();
     h->free_rs();
     h->free_comm();
     h->free_caph();
@@ -1240,7 +1250,7 @@ StepIO md_io(vb_handle* h) {
     io.ef = h->md_ef;
     return io;
 }
-// fragment placement -> evaluation + signed whole-protein reduction [-> non-bonded term] [-> restraints], all on st
+// fragment placement -> evaluation + signed whole-protein reduction [-> MM or PME non-bonded term] [-> restraints], all on st
 int md_eval_enqueue(vb_handle* h, cudaStream_t st) {
     const int N = h->ws.N;
     md_place_kernel<<<(N + 255) / 256, 256, 0, st>>>(N, h->d_real, h->d_acc, h->d_rem, h->d_blen, h->d_mx, h->d_pos);
@@ -1250,6 +1260,7 @@ int md_eval_enqueue(vb_handle* h, cudaStream_t st) {
         nonbonded_kernel<double><<<(h->nb.hi - h->nb.lo + 7) / 8, 256, 0, st>>>(h->nb, h->d_mx, h->md_ef, h->d_nb_eatom);
         nonbonded_energy_kernel<<<1, 256, 0, st>>>(h->nb, h->d_nb_eatom, h->md_ef);
     }
+    if (h->pme_ready) pme_launch<double>(h->pme, h->d_mx, h->md_ef, st);   // PME non-bonded term instead
     if (h->rs_ready && h->rs.hi > h->rs.lo)         // Hookean restraints on the same protein coordinates
         restraint_kernel<<<1, RS_THREADS, 0, st>>>(h->rs, h->d_mx, h->md_ef);
     CUDA_TRY(h, cudaGetLastError());
@@ -1417,6 +1428,32 @@ int vb_md_get_state(vb_handle* h, double* x_host, double* v_host, int64_t* step_
 
 
 // ---- non-bonded MM term (k_nonbonded.cuh) ----------------------------------------------------------------
+namespace {
+// CSR exclusion table over P atoms: rowptr[0] = 0, monotone, every row strictly ascending indices in [0, P)
+int check_exclusions(vb_handle* h, const char* who, int P, const int32_t* rowptr, const int32_t* col) {
+    const int64_t nx = rowptr[P];
+    if (rowptr[0] != 0 || nx < 0 || (nx > 0 && !col)) { h->set_error("%s: bad exclusion table", who); return VB_ERR_ARG; }
+    for (int i = 0; i < P; i++) {
+        if (rowptr[i + 1] < rowptr[i]) { h->set_error("%s: exclusion row pointer not monotone", who); return VB_ERR_ARG; }
+        for (int k = rowptr[i]; k < rowptr[i + 1]; k++) {
+            const int c = col[k];
+            if (c < 0 || c >= P || (k > rowptr[i] && c <= col[k - 1])) {
+                h->set_error("%s: exclusion row %d must be strictly ascending atom indices", who, i);
+                return VB_ERR_ARG;
+            }
+        }
+    }
+    return VB_OK;
+}
+// ASE 3.22 unit system (CODATA 2014): nonbonded.py:18 / pme.py:120 k = 1/(4 pi eps0) * 10e6 * mol * C^-2 ; kJ/mol in eV
+void coulomb_units(double* k, double* kj_mol) {
+    const double c = 299792458.0, mu0 = 4.0e-7 * 3.14159265358979323846, eps0 = 1.0 / mu0 / (c * c);
+    const double e_ch = 1.6021766208e-19, nav = 6.022140857e23, coul = 1.0 / e_ch, kj = 1000.0 / e_ch;
+    *k = 1.0 / (4.0 * 3.14159265358979323846 * eps0) * 10e6 * nav / (coul * coul);
+    *kj_mol = kj / nav;
+}
+}  // namespace
+
 int vb_set_nonbonded(vb_handle* h, int64_t n_protein_atoms, const float* charges_host, const float* sigmas_nm_host,
                      const float* epsilons_kj_host, const int32_t* excl_rowptr_host, const int32_t* excl_col_host,
                      int64_t atom_lo, int64_t atom_hi) {
@@ -1433,18 +1470,12 @@ int vb_set_nonbonded(vb_handle* h, int64_t n_protein_atoms, const float* charges
     }
     const int P = (int)n_protein_atoms;
     const int64_t nx = excl_rowptr_host[P];
-    if (excl_rowptr_host[0] != 0 || nx < 0 || (nx > 0 && !excl_col_host)) { h->set_error("vb_set_nonbonded: bad exclusion table"); return VB_ERR_ARG; }
-    for (int i = 0; i < P; i++) {
-        if (excl_rowptr_host[i + 1] < excl_rowptr_host[i]) { h->set_error("vb_set_nonbonded: exclusion row pointer not monotone"); return VB_ERR_ARG; }
-        for (int k = excl_rowptr_host[i]; k < excl_rowptr_host[i + 1]; k++) {
-            const int c = excl_col_host[k];
-            if (c < 0 || c >= P || (k > excl_rowptr_host[i] && c <= excl_col_host[k - 1])) {
-                h->set_error("vb_set_nonbonded: exclusion row %d must be strictly ascending atom indices", i);
-                return VB_ERR_ARG;
-            }
-        }
-    }
+    if (int rc = check_exclusions(h, "vb_set_nonbonded", P, excl_rowptr_host, excl_col_host)) return rc;
     CUDA_TRY(h, cudaSetDevice(h->device));
+    if (h->pme_ready) {                 // one non-bonded term at a time; MD graph replays may still read the PME arrays
+        CUDA_TRY(h, cudaDeviceSynchronize());
+        h->free_pme();
+    }
     h->drop_graph();
     h->free_nb();
     CUDA_TRY(h, cudaMalloc(&h->d_nb_q, sizeof(float) * P));
@@ -1459,12 +1490,10 @@ int vb_set_nonbonded(vb_handle* h, int64_t n_protein_atoms, const float* charges
     CUDA_TRY(h, cudaMemcpy(h->d_nb_rowptr, excl_rowptr_host, sizeof(int) * (P + 1), cudaMemcpyHostToDevice));
     if (nx > 0) CUDA_TRY(h, cudaMemcpy(h->d_nb_col, excl_col_host, sizeof(int) * nx, cudaMemcpyHostToDevice));
     CUDA_TRY(h, cudaMemset(h->d_nb_eatom, 0, sizeof(double) * P));
-    // ASE 3.22 unit system (CODATA 2014): nonbonded.py:18 k = 1/(4 pi eps0) * 10e6 * mol * C^-2 ; kJ/mol in eV
-    const double c = 299792458.0, mu0 = 4.0e-7 * 3.14159265358979323846, eps0 = 1.0 / mu0 / (c * c);
-    const double e_ch = 1.6021766208e-19, nav = 6.022140857e23, coul = 1.0 / e_ch, kj = 1000.0 / e_ch;
-    const double k = 1.0 / (4.0 * 3.14159265358979323846 * eps0) * 10e6 * nav / (coul * coul);
+    double k, kj_mol;
+    coulomb_units(&k, &kj_mol);
     h->nb = NbParams{P, (int)atom_lo, (int)atom_hi, h->d_nb_q, h->d_nb_sigma, h->d_nb_eps, h->d_nb_rowptr, h->d_nb_col,
-                     (float)k, (float)(kj / nav)};
+                     (float)k, (float)kj_mol};
     h->nb_ready = true;
     return VB_OK;
 }
@@ -1484,6 +1513,113 @@ int vb_nonbonded(vb_handle* h, const float* prot_pos_dev, float* ef_prot_dev, vo
     return VB_OK;
 }
 
+
+// ---- PME non-bonded term (k_pme.cuh) -------------------------------------------------------------------------------
+int vb_set_pme(vb_handle* h, const vb_pme_params* pp) {
+    if (!h) return VB_ERR_ARG;
+    std::lock_guard<std::mutex> lk(h->mu);
+    auto bad = [&](const char* what) { h->set_error("vb_set_pme: %s", what); return VB_ERR_ARG; };
+    if (!pp) return bad("null parameters");
+    const int64_t n = pp->n_protein_atoms;
+    if (n <= 0 || n > (1 << 24) || !pp->charges || !pp->sigmas_nm || !pp->epsilons_kj || !pp->excl_rowptr)
+        return bad("bad arguments");
+    if (pp->atom_lo < 0 || pp->atom_hi < pp->atom_lo || pp->atom_hi > n) return bad("bad slice: [atom_lo, atom_hi) must lie in [0, n)");
+    if (h->n_protein > 0 && h->n_protein != n) return bad("n_protein_atoms differs from the protein map's");
+    for (int a = 0; a < 3; a++) {
+        if (!std::isfinite(pp->cell[a]) || !(pp->cell[a] > 0.0)) return bad("cell lengths must be finite and positive");
+        if (pp->grid[a] < 4) return bad("grid dimensions must be at least 4 (spline order)");
+        if (pp->grid[a] > 4096) return bad("grid dimensions must be at most 4096");
+    }
+    if ((int64_t)pp->grid[0] * pp->grid[1] * pp->grid[2] > (1LL << 27)) return bad("grid has more than 2^27 points");
+    if (!std::isfinite(pp->beta) || !(pp->beta > 0.0)) return bad("beta must be finite and positive");
+    if (!std::isfinite(pp->cutoff) || !(pp->cutoff > 0.0)) return bad("cutoff must be finite and positive");
+    const int P = (int)n;
+    if (int rc = check_exclusions(h, "vb_set_pme", P, pp->excl_rowptr, pp->excl_col)) return rc;
+    const int64_t nx = pp->excl_rowptr[P];
+    const int K1 = pp->grid[0], K2 = pp->grid[1], K3 = pp->grid[2], H3 = K3 / 2 + 1;
+    // host tables: per-axis twiddles cos / sin(2 pi j / K) and B-spline moduli 36 / (4 + 2 cos(2 pi m / K))^2
+    std::vector<double> tw, bmod;
+    for (int K : {K1, K2, K3})
+        for (int j = 0; j < K; j++) {
+            const double th = 2.0 * 3.14159265358979323846 * j / K;
+            tw.push_back(cos(th)); tw.push_back(sin(th));
+            bmod.push_back(36.0 / ((4.0 + 2.0 * cos(th)) * (4.0 + 2.0 * cos(th))));
+        }
+    double qsum = 0.0, q2 = 0.0;
+    for (int i = 0; i < P; i++) { qsum += pp->charges[i]; q2 += (double)pp->charges[i] * pp->charges[i]; }
+    const float qtot = (float)qsum, zero_pos[3] = {0.f, 0.f, 0.f};
+    // MD graph replays enqueued before this call may still read the old arrays
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    CUDA_TRY(h, cudaDeviceSynchronize());
+    h->drop_graph();
+    h->free_nb();                       // one non-bonded term at a time (FragmentCalculator's nonbonded_calcs[type])
+    h->free_pme();
+    struct Piece { const void* src; size_t bytes; size_t off; };
+    std::vector<Piece> pieces;
+    size_t total = 0;
+    auto add = [&](const void* src, size_t bytes) {
+        pieces.push_back({src, bytes, total});
+        total += (std::max<size_t>(bytes, 8) + 255) & ~(size_t)255;
+        return pieces.size() - 1;
+    };
+    const size_t nh = (size_t)K1 * K2 * H3, ngrid = (size_t)K1 * K2 * K3;
+    const int n_partial = (int)((nh + PME_THREADS - 1) / PME_THREADS);
+    const size_t i_q = add(pp->charges, 4 * (size_t)P), i_s = add(pp->sigmas_nm, 4 * (size_t)P), i_e = add(pp->epsilons_kj, 4 * (size_t)P);
+    const size_t i_rp = add(pp->excl_rowptr, 4 * (size_t)(P + 1)), i_cl = add(nx > 0 ? pp->excl_col : nullptr, 4 * (size_t)nx);
+    const size_t i_tw = add(tw.data(), 8 * tw.size()), i_bm = add(bmod.data(), 8 * bmod.size());
+    const size_t i_base = add(nullptr, 12 * (size_t)P), i_w = add(nullptr, 96 * (size_t)P);
+    const size_t i_bp = add(nullptr, 4 * (size_t)(K1 + 1)), i_ba = add(nullptr, 4 * (size_t)P);
+    const size_t i_Q = add(nullptr, 8 * ngrid), i_A = add(nullptr, 16 * nh), i_B = add(nullptr, 16 * nh);
+    const size_t i_pa = add(nullptr, 8 * (size_t)n_partial), i_ea = add(nullptr, 8 * (size_t)PME_NATOM * P);
+    const size_t i_t = add(nullptr, 8 * PT_N);
+    const size_t i_zp = add(zero_pos, sizeof(zero_pos)), i_qt = add(&qtot, 4), i_ef1 = add(nullptr, 16);
+    CUDA_TRY(h, cudaMalloc(&h->pme_mem, total));
+    char* base = static_cast<char*>(h->pme_mem);
+    CUDA_TRY(h, cudaMemset(base, 0, total));
+    for (const Piece& pc : pieces)
+        if (pc.src && pc.bytes) CUDA_TRY(h, cudaMemcpy(base + pc.off, pc.src, pc.bytes, cudaMemcpyHostToDevice));
+    auto at = [&](size_t i) { return static_cast<void*>(base + pieces[i].off); };
+    double k, kj_mol;
+    coulomb_units(&k, &kj_mol);
+    PmeParams& m = h->pme;
+    m = PmeParams{};
+    m.n = P; m.lo = (int)pp->atom_lo; m.hi = (int)pp->atom_hi; m.recip = pp->atom_lo == 0;
+    m.q = (const float*)at(i_q); m.sigma = (const float*)at(i_s); m.eps = (const float*)at(i_e);
+    m.excl_rowptr = (const int*)at(i_rp); m.excl_col = (const int*)at(i_cl);
+    m.coulomb_k = (float)k; m.kj_mol = (float)kj_mol;
+    m.beta = (float)pp->beta; m.rc2 = (float)pp->cutoff * (float)pp->cutoff;
+    m.beta64 = pp->beta; m.k64 = k; m.kj64 = kj_mol;
+    m.K1 = K1; m.K2 = K2; m.K3 = K3; m.H3 = H3;
+    m.L1 = pp->cell[0]; m.L2 = pp->cell[1]; m.L3 = pp->cell[2];
+    m.tw = (const double*)at(i_tw); m.bmod = (const double*)at(i_bm);
+    m.base = (int*)at(i_base); m.w = (double*)at(i_w); m.bin_ptr = (int*)at(i_bp); m.bin_atom = (int*)at(i_ba);
+    m.Q = (double*)at(i_Q); m.A = (double2*)at(i_A); m.B = (double2*)at(i_B);
+    m.partial = (double*)at(i_pa); m.eatom = (double*)at(i_ea); m.terms = (double*)at(i_t);
+    // electro_neutral (pme.py:99-110): the same kernels on one particle of charge q_tot at the origin give its E_rec
+    PmeParams one = m;
+    one.n = 1; one.lo = one.hi = 0; one.recip = true; one.q = (const float*)at(i_qt);
+    pme_launch<float>(one, (const float*)at(i_zp), (float*)at(i_ef1), h->own_stream);
+    double rec1 = 0.0;
+    CUDA_TRY(h, cudaGetLastError());
+    CUDA_TRY(h, cudaStreamSynchronize(h->own_stream));
+    CUDA_TRY(h, cudaMemcpy(&rec1, m.terms + PT_REC, sizeof(double), cudaMemcpyDeviceToHost));
+    const double sqpi = sqrt(3.14159265358979323846);
+    m.slf = -pp->beta / sqpi * q2;                                          // electro_slf, pme.py:86-87
+    m.neutral = -rec1 + pp->beta * qsum * qsum / sqpi;                     // E_rec of fp32 q_tot (helpmelib.MatrixF)
+    h->pme_ready = true;
+    return VB_OK;
+}
+
+int vb_pme(vb_handle* h, const float* prot_pos_dev, float* ef_prot_dev, void* stream) {
+    if (!h) return VB_ERR_ARG;
+    std::lock_guard<std::mutex> lk(h->mu);
+    if (!h->pme_ready) { h->set_error("vb_pme: call vb_set_pme first"); return VB_ERR_STATE; }
+    if (!prot_pos_dev || !ef_prot_dev) { h->set_error("vb_pme: null buffer"); return VB_ERR_ARG; }
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    pme_launch<float>(h->pme, prot_pos_dev, ef_prot_dev, (cudaStream_t)stream);
+    CUDA_TRY(h, cudaGetLastError());
+    return VB_OK;
+}
 
 // ---- Hookean restraints (k_restraint.cuh) ------------------------------------------------------------------------
 int vb_set_restraints(vb_handle* h, const vb_restraint_set* rs) {
@@ -1826,6 +1962,7 @@ int64_t vb_get_option(const vb_handle* h, const char* key) {
     }
     if (k == "comm_ready") return h->comm_ready ? 1 : 0;
     if (k == "restraints_ready") return h->rs_ready ? 1 : 0;
+    if (k == "pme_ready") return h->pme_ready ? 1 : 0;
     if (k == "edge_overflow") {
         int flag = 0;
         if (h->d_flags && cudaMemcpy(&flag, h->d_flags, sizeof(int), cudaMemcpyDeviceToHost) != cudaSuccess) return VB_ERR_CUDA;
@@ -1923,6 +2060,16 @@ int vb_tc_selftest(int device, const float* a_host, const float* img_host, float
 int64_t vb_debug_read(vb_handle* h, const char* name, int layer, void* host_dst, int64_t cap_bytes) {
     if (!h || !name || !host_dst) return VB_ERR_ARG;
     std::lock_guard<std::mutex> lk(h->mu);
+    if (std::string(name) == "pme_terms") {              // needs no topology: the PME term stands on its own
+        if (!h->pme_ready) { h->set_error("vb_debug_read: pme_terms: no PME term set"); return VB_ERR_STATE; }
+        const int64_t bytes = std::min<int64_t>(cap_bytes, sizeof(double) * PT_N);
+        if (cudaSetDevice(h->device) != cudaSuccess || cudaDeviceSynchronize() != cudaSuccess ||
+            cudaMemcpy(host_dst, h->pme.terms, bytes, cudaMemcpyDeviceToHost) != cudaSuccess) {
+            h->set_error("vb_debug_read: copy failed: %s", cudaGetErrorString(cudaGetLastError()));
+            return VB_ERR_CUDA;
+        }
+        return bytes;
+    }
     if (!h->has_topology) return VB_ERR_STATE;
     const Workspace& ws = h->ws;
     const size_t N = ws.N, E = ws.Ecap, G = ws.G;

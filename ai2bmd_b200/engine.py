@@ -40,13 +40,20 @@ class _RestraintSet(C.Structure):
                 ("pair_rt", C.c_void_p), ("atom_lo", C.c_int64), ("atom_hi", C.c_int64)]
 
 
+class _PmeParams(C.Structure):
+    _fields_ = [("n_protein_atoms", C.c_int64), ("charges", C.c_void_p), ("sigmas_nm", C.c_void_p),
+                ("epsilons_kj", C.c_void_p), ("excl_rowptr", C.c_void_p), ("excl_col", C.c_void_p),
+                ("cell", C.c_double * 3), ("grid", C.c_int32 * 3), ("beta", C.c_double), ("cutoff", C.c_double),
+                ("atom_lo", C.c_int64), ("atom_hi", C.c_int64)]
+
+
 # every symbol include/visnet_b200.h declares (tests check that the library exports each of them)
 EXPORTED_SYMBOLS = [
     "vb_weight_manifest", "vb_create", "vb_destroy", "vb_last_error", "vb_set_topology", "vb_forward",
     "vb_forward_host", "vb_set_protein_map", "vb_forward_protein", "vb_get_edges", "vb_launches_per_forward",
     "vb_set_option", "vb_get_option", "vb_num_stages", "vb_stage_name", "vb_debug_run", "vb_debug_read", "vb_profile_stages", "vb_tc_selftest",
     "vb_md_setup", "vb_md_set_normals", "vb_md_set_state", "vb_md_kick1", "vb_md_eval", "vb_md_kick2", "vb_md_run", "vb_md_get_state",
-    "vb_set_nonbonded", "vb_nonbonded", "vb_set_restraints", "vb_restraints",
+    "vb_set_nonbonded", "vb_nonbonded", "vb_set_pme", "vb_pme", "vb_set_restraints", "vb_restraints",
     "vb_comm_init", "vb_comm_connect", "vb_comm_allreduce",
     "vb_set_caph", "vb_caph_relax",
 ]
@@ -116,6 +123,10 @@ def load_library(path: Optional[str] = None):
     lib.vb_set_nonbonded.argtypes = [vp, i64, vp, vp, vp, vp, vp, i64, i64]
     lib.vb_nonbonded.restype = C.c_int
     lib.vb_nonbonded.argtypes = [vp, vp, vp, vp]
+    lib.vb_set_pme.restype = C.c_int
+    lib.vb_set_pme.argtypes = [vp, C.POINTER(_PmeParams)]
+    lib.vb_pme.restype = C.c_int
+    lib.vb_pme.argtypes = [vp, vp, vp, vp]
     lib.vb_set_restraints.restype = C.c_int
     lib.vb_set_restraints.argtypes = [vp, C.POINTER(_RestraintSet)]
     lib.vb_restraints.restype = C.c_int
@@ -283,6 +294,37 @@ class Engine:
 
     def nonbonded_device(self, prot_pos_ptr: int, ef_ptr: int, stream_ptr: int = 0):
         self._check(self.lib.vb_nonbonded(self.h, prot_pos_ptr, ef_ptr, stream_ptr), "vb_nonbonded")
+
+    # ---- PME non-bonded term (include/visnet_b200.h: vb_set_pme / vb_pme) ----
+    def set_pme(self, charges, sigmas_nm, epsilons_kj, excl_rowptr, excl_col, cell, grid, beta: float = 0.3,
+                cutoff: float = 9.0, atom_lo: int = 0, atom_hi: int = -1):
+        """Install the PME non-bonded term (replaces the MM term if one is set).  ``cell``: orthorhombic lengths (A),
+        ``grid``: mesh points per axis; ``atom_hi < 0`` means every atom."""
+        q = np.ascontiguousarray(charges, dtype=np.float32)
+        sg = np.ascontiguousarray(sigmas_nm, dtype=np.float32)
+        ep = np.ascontiguousarray(epsilons_kj, dtype=np.float32)
+        rp = np.ascontiguousarray(excl_rowptr, dtype=np.int32)
+        cl = np.ascontiguousarray(excl_col, dtype=np.int32)
+        n = len(q)
+        if not (len(sg) == len(ep) == n and len(rp) == n + 1 and int(rp[-1]) == len(cl)):
+            raise ValueError("non-bonded parameter arrays / exclusion table have inconsistent lengths")
+        if len(cell) != 3 or len(grid) != 3:
+            raise ValueError("cell and grid need three entries")
+        p = _PmeParams(n, q.ctypes.data, sg.ctypes.data, ep.ctypes.data, rp.ctypes.data, cl.ctypes.data if len(cl) else None,
+                       (C.c_double * 3)(*[float(c) for c in cell]), (C.c_int32 * 3)(*[int(k) for k in grid]),
+                       float(beta), float(cutoff), int(atom_lo), int(n if atom_hi < 0 else atom_hi))
+        self._check(self.lib.vb_set_pme(self.h, C.byref(p)), "vb_set_pme")
+
+    def pme_device(self, prot_pos_ptr: int, ef_ptr: int, stream_ptr: int = 0):
+        """ef[3n+1] += PME forces / energy at the fp32 protein positions (device pointers); asynchronous."""
+        self._check(self.lib.vb_pme(self.h, prot_pos_ptr, ef_ptr, stream_ptr), "vb_pme")
+
+    def pme_terms(self) -> Dict[str, float]:
+        """fp64 terms of the last PME evaluation (synchronises): E_dir, E_adj, E_ex, E_rec, slf, neutral in e^2/A,
+        E_LJ, E_LJ_ex in kJ/mol (E_dir / E_LJ: non-excluded pairs inside the cutoff, E_ex / E_LJ_ex: excluded pairs
+        beyond it)."""
+        t = self.debug_read("pme_terms", 0, (8,), np.float64)
+        return dict(zip(("E_dir", "E_adj", "E_ex", "E_rec", "slf", "neutral", "E_LJ", "E_LJ_ex"), t.tolist()))
 
     # ---- Hookean restraints (include/visnet_b200.h: vb_set_restraints / vb_restraints) ----
     def set_restraints(self, point_atom=(), point_anchor=(), point_k=(), point_rt=(), pair_ij=(), pair_k=(), pair_rt=(),

@@ -1,4 +1,5 @@
-"""Host side of the non-bonded MM term -- mirror of ``MMNonBondedCalculator`` (``src/Calculators/nonbonded.py:9-63``).
+"""Host side of the non-bonded terms -- mirrors of ``MMNonBondedCalculator`` (``src/Calculators/nonbonded.py:9-63``)
+and ``PMENonBondedCalculator`` (``src/Calculators/pme.py:113-214``), the two choices of ``--fragment-longrange-calc``.
 
 The reference obtains per-atom charges / sigmas / epsilons from OpenMM's amber14 force field
 (``src/AIMD/protein.py:153-175``); OpenMM is not part of this image, so the parameters are inputs here, in the
@@ -69,6 +70,46 @@ class MMNonBondedCalculator:
         self.pos.copy_(torch.from_numpy(p), non_blocking=True)
         self.ef.zero_()
         self.engine.nonbonded_device(self.pos.data_ptr(), self.ef.data_ptr(), stream.cuda_stream)
+        ef = self.ef.cpu().numpy()
+        return float(ef[-1]), ef[:-1].reshape(-1, 3).copy()
+
+
+class PMENonBondedCalculator:
+    """Mirror of the reference's ``PMENonBondedCalculator`` (``src/Calculators/pme.py:113-214``) on the device:
+    ``set_parameters`` once, then ``calc(positions) -> (energy [eV], forces [n,3] eV/A)`` per step."""
+
+    def __init__(self, engine: Engine, beta: float = 0.3, cutoff: float = 9.0, grid_spacing: float = 1.0):
+        import torch
+        self.torch = torch
+        self.engine = engine
+        self.beta, self.cutoff, self.grid_spacing = float(beta), float(cutoff), float(grid_spacing)
+        self.n = 0
+
+    def grid(self, cell) -> Tuple[int, int, int]:
+        """Mesh points per axis, ``int(cell_len / grid_spacing)`` (pme.py:146-149)."""
+        return tuple(int(c / self.grid_spacing) for c in cell)
+
+    def set_parameters(self, charges, sigmas_nm, epsilons_kj, excl_rowptr, excl_col, cell, atom_lo: int = 0,
+                       atom_hi: int = -1):
+        """``cell``: the orthorhombic cell lengths (A), e.g. :func:`ai2bmd_b200.pdbfrag.read_cell` of the input PDB."""
+        torch = self.torch
+        cell = tuple(float(c) for c in cell)
+        self.engine.set_pme(charges, sigmas_nm, epsilons_kj, excl_rowptr, excl_col, cell, self.grid(cell), self.beta,
+                            self.cutoff, atom_lo, atom_hi)
+        self.n = len(charges)
+        dev = torch.device("cuda", self.engine.device)
+        self.pos = torch.empty((self.n, 3), dtype=torch.float32, device=dev)
+        self.ef = torch.empty(3 * self.n + 1, dtype=torch.float32, device=dev)
+
+    def __call__(self, positions) -> Tuple[float, np.ndarray]:
+        torch = self.torch
+        p = np.ascontiguousarray(positions, dtype=np.float32)        # pme.py:162 casts to fp32
+        if p.shape != (self.n, 3):
+            raise ValueError(f"positions must be [{self.n}, 3]")
+        stream = torch.cuda.current_stream(self.pos.device)
+        self.pos.copy_(torch.from_numpy(p), non_blocking=True)
+        self.ef.zero_()
+        self.engine.pme_device(self.pos.data_ptr(), self.ef.data_ptr(), stream.cuda_stream)
         ef = self.ef.cpu().numpy()
         return float(ef[-1]), ef[:-1].reshape(-1, 3).copy()
 

@@ -24,7 +24,7 @@ reports the margin, and the AMBER order of a dipeptide is available through ``ai
 from __future__ import annotations
 
 from dataclasses import dataclass
-from typing import List
+from typing import List, Tuple
 
 import numpy as np
 
@@ -61,6 +61,21 @@ def read_pdb(path: str) -> CappedProtein:
     resi = np.asarray(resi)
     resi = resi - resi.min() + 1
     return CappedProtein(names, resn, resi, elem, np.asarray(xyz, dtype=np.float64))
+
+
+def read_cell(path: str) -> Tuple[float, float, float]:
+    """Cell lengths a, b, c (A) of the PDB's ``CRYST1`` record -- the cell the reference's PME term uses
+    (``pme.py:146``, an orthorhombic ``XAligned`` lattice).  Raises ``ValueError`` when the record is missing or an
+    angle is not 90 degrees."""
+    with open(path) as fh:
+        for line in fh:
+            if line.startswith("CRYST1"):
+                a, b, c = float(line[6:15]), float(line[15:24]), float(line[24:33])
+                angles = (float(line[33:40]), float(line[40:47]), float(line[47:54]))
+                if any(abs(x - 90.0) > 1e-6 for x in angles):
+                    raise ValueError(f"{path}: CRYST1 angles {angles} are not all 90 degrees (PME needs an orthorhombic cell)")
+                return a, b, c
+    raise ValueError(f"{path}: no CRYST1 record (PME needs the cell)")
 
 
 @dataclass

@@ -84,7 +84,7 @@ int vb_forward_protein(vb_handle* h, const float* pos_dev, float* ef_prot_dev, v
 
 /* ---- Device-resident MD step (SURVEY section 8f, rank 3 and the first half of rank 1) ------------------------
  * State (protein positions / velocities, fp64) stays on the GPU; one step is
- *   kick1 (half-kick + drift) -> eval (place fragment atoms, ViSNet, signed reduction into ef [+ non-bonded term]
+ *   kick1 (half-kick + drift) -> eval (place fragment atoms, ViSNet, signed reduction into ef [+ MM or PME non-bonded term]
  *   [+ restraints]) -> kick2.
  * Replaces: the ASE Langevin loop the reference runs (src/AIMD/simulator.py:96-137: Langevin(dt = 1 fs, 300 K,
  *           friction 0.001/fs), MaxwellBoltzmannDistribution start; ASE 3.22 ase/md/langevin.py step()) and the
@@ -133,6 +133,39 @@ int vb_set_nonbonded(vb_handle* h, int64_t n_protein_atoms, const float* charges
  * bonded + non-bonded (FragmentCalculator.calculate, src/Calculators/fragment.py:50-68).  Once set, vb_md_eval
  * adds the term too. */
 int vb_nonbonded(vb_handle* h, const float* prot_pos_dev, float* ef_prot_dev, void* stream);
+
+/* ---- PME non-bonded term (the reference's --fragment-longrange-calc pme) ---------------------------------------------
+ *   E = [k (E_rec + E_dir + E_adj + slf + neutral - E_ex) + E_LJ - E_LJ_ex] * kJ/mol,  F = sum_P (F_LJ + F_C) - sum_X (F_LJ + F_C)
+ * P: ordered pairs i != j closer than `cutoff` (no periodic images; pairs inside a dipeptide included), X: the pairs of
+ * the exclusion table (atoms sharing a dipeptide), every pair sum halved.  E_dir / E_ex: q_i q_j erfc(beta d) / d over P / X,
+ * E_adj: -q_i q_j erf(beta d) / d over X, E_rec: smooth PME reciprocal energy (order-4 B-splines on a grid[0] x grid[1] x
+ * grid[2] mesh of the orthorhombic cell, fp64), slf = -beta / sqrt(pi) sum q^2, neutral = -E_rec(q_tot at the origin) +
+ * beta q_tot^2 / sqrt(pi).  F_C = k q_i q_j vec / d^3 is the plain Coulomb force and E_rec contributes no force, as in the
+ * reference.  A pair in both P and X contributes its net value (only its erf term), not a difference of fp32 sums.
+ * Replaces: PMENonBondedCalculator.set_parameters / __call__, src/Calculators/pme.py:132-214 (beta 0.3, cutoff 9 A,
+ *           grid int(cell / 1 A)).  Host helpers: ai2bmd_b200/nonbonded.py PMENonBondedCalculator, pdbfrag.read_cell. */
+typedef struct {
+    int64_t n_protein_atoms;
+    const float* charges; const float* sigmas_nm; const float* epsilons_kj;   /* as vb_set_nonbonded */
+    const int32_t* excl_rowptr; const int32_t* excl_col;                       /* as vb_set_nonbonded */
+    double cell[3];           /* orthorhombic cell lengths, Angstrom */
+    int32_t grid[3];          /* mesh points per axis, >= 4 */
+    double beta;              /* Ewald screening parameter, 1/Angstrom */
+    double cutoff;            /* real-space cutoff, Angstrom */
+    int64_t atom_lo, atom_hi; /* destination atoms of the direct sums; the slice with atom_lo == 0 adds E_rec and the constants */
+} vb_pme_params;
+/* Host pointers, copied.  VB_ERR_ARG for a non-finite or non-positive cell length, beta or cutoff, a grid dimension
+ * below 4 (or above 4096, or more than 2^27 points), a bad exclusion table or slice, or n_protein_atoms other than the
+ * protein map's.  Replaces the MM term if one is set (and vb_set_nonbonded replaces this one): the handle holds at most
+ * one non-bonded term.  Synchronises the device; captured graphs are dropped.  Computes `neutral` with the reciprocal
+ * kernels on a one-particle input.  Once set, vb_md_eval / vb_md_run add the term where the MM term goes. */
+int vb_set_pme(vb_handle* h, const vb_pme_params* params);
+/* ef_prot_dev[3*n + 1] += PME forces / energy at prot_pos_dev[n*3] (fp32 positions as the reference casts them,
+ * pme.py:162).  Accumulates.  Two calls on the same input give bit-identical results (no atomics).
+ * vb_debug_read("pme_terms") returns the fp64 terms of the last evaluation: E_dir, E_adj, E_ex, E_rec, slf, neutral
+ * (e^2/Angstrom) and E_LJ, E_LJ_ex (kJ/mol); E_dir / E_LJ cover the non-excluded pairs inside the cutoff and E_ex /
+ * E_LJ_ex the excluded pairs beyond it, which have the reference's differences E_dir - E_ex and E_LJ - E_LJ_ex. */
+int vb_pme(vb_handle* h, const float* prot_pos_dev, float* ef_prot_dev, void* stream);
 
 /* ---- Hookean restraints (pre-equilibration and hydrogen-bond constraints) ------------------------------------------
  * point (a, p0, k, rt): d = p0 - x_a, r = |d|; if r > rt: F_a += k (r - rt) d/r, E += k (r - rt)^2 / 2.
@@ -215,7 +248,7 @@ int vb_launches_per_forward(const vb_handle* h);
  * different row (default 1: the CTAs of a wave otherwise ask the same L2 slices for the same rows at the same time),
  * "embed_batch" -1/0..3 batch variants of the embedding kernels, "comm_auto" 0/1.  vb_get_option also answers "edge_overflow" (1 after a step exceeded a trimmed max_edges),
  * "tile_rows" (planned edges per tile), "comm_ready", "caph_ready", "caph_evals" (energy evaluations of the last hydrogen refinement)
- * and "restraints_ready" (1 while a non-empty restraint set is installed). */
+ * "restraints_ready" (1 while a non-empty restraint set is installed) and "pme_ready" (1 while the PME term is installed). */
 int vb_set_option(vb_handle* h, const char* key, int64_t value);
 int64_t vb_get_option(const vb_handle* h, const char* key);   /* resolved value (after vb_set_topology) */
 
@@ -232,7 +265,7 @@ int vb_profile_stages(vb_handle* h, const float* pos_dev, int n_iter, float* ms_
 int vb_tc_selftest(int device, const float* a_host, const float* img_host, float* d_host, int reps, float* ms_out);
 /* Copy an internal buffer to the host.  name: "X","V","F","VN","QKV","V123","VDOT","TU","O" (per layer),
  * "XA","VA","GX","GVEC","GF","GXA","GQKV","GVNMSG","GTU","GQKV2","GVNMSG2","GTU2","geom","rbf","eacc","grbf","esrc","edst","rowptr",
- * "eatom","energy","forces".  Returns the number of bytes copied (<= cap_bytes) or a negative status. */
+ * "eatom","energy","forces", "pme_terms" (8 doubles, see vb_pme).  Returns the number of bytes copied (<= cap_bytes) or a negative status. */
 int64_t vb_debug_read(vb_handle* h, const char* name, int layer, void* host_dst, int64_t cap_bytes);
 
 #ifdef __cplusplus
